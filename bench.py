@@ -2,6 +2,7 @@
 """bench.py -- throughput of the conv hot path (convertWithModels) on B200, one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size S] [--engine auto|tc|fp32]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json config 3, the one the metric is quoted on): one full scale2.0x model pass
 (7 layers, 574 272 algorithmic FLOP per output pixel) over a synthetic 4096x4096 fp32 Y plane.
@@ -284,6 +285,25 @@ def host_api_legs(w2x, steps, size):
 
 
 
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, plane, rank, world):
+    """Write the output plane of the timed path's last step as <out_dir>/output.npy (float32), so that two builds can be
+    compared output for output on the same seeded input.  A plane larger than this rank's share of DUMP_BYTES is cut to
+    a fixed, seeded sample of whole rows; output_rows.npy (float64) lists which rows, in order.  With N > 1 ranks every
+    rank writes its band as output_rank<r>.npy / output_rows_rank<r>.npy."""
+    import torch
+    h, w = plane.shape
+    keep = min(h, max(1, DUMP_BYTES // world // (w * 4)))
+    rows = np.arange(h) if keep == h else np.sort(np.random.default_rng(0).choice(h, size=keep, replace=False))
+    sample = plane.index_select(0, torch.as_tensor(rows, device=plane.device)).cpu().numpy().astype(np.float32)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"output{suffix}.npy"), sample)
+    np.save(os.path.join(out_dir, f"output_rows{suffix}.npy"), rows.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -437,6 +457,8 @@ def run_ours(args):
         halo_check = True
     sampler = ClockSampler(local) if rank == 0 else None
     ms_dev, _, launches, layers, clocks = timed(step_device, args.steps, with_layers=True, sampler=sampler)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_out, rank, world)
     for _ in range(min(args.warmup, 2)):
         step_e2e()
     _, ms_e2e_wall, _, _, _ = timed(step_e2e, args.steps)
@@ -591,7 +613,11 @@ def main():
                          "the same rows through torch.distributed send/recv, or 7 input rows once (recompute)")
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg4 (8192^2 strong) and cfg5 (64 tiles) legs")
     ap.add_argument("--cfg4-size", type=int, default=8192)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output plane of the last one to DIR/output.npy (a seeded row sample above 32 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

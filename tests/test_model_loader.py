@@ -1,15 +1,12 @@
 """Host side of the boundary: JSON model loader (w2x_model_load_json), in-memory constructor and the
 tcgen05 operand packing.  No GPU needed."""
-import hashlib
 import json
-import os
 
 import numpy as np
 import pytest
 
 from conftest import golden_path
-
-REF_MODELS = "/root/reference/models"
+from oracle import reference_golden as RG
 
 
 def test_load_json_roundtrip_matches_golden_params(w2x, oracle_models, json_models):
@@ -24,17 +21,22 @@ def test_load_json_roundtrip_matches_golden_params(w2x, oracle_models, json_mode
             assert np.array_equal(b, om.biases[li])        # biases stay double
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MODELS), reason="reference checkout not present (GPU box)")
-def test_load_reference_json_files_known_answers(w2x, oracle_models):
+def test_load_reference_json_files_known_answers(w2x, oracle_models, tmp_path):
+    """The first and last layer of each shipped model file, spelt as the reference ships them (tests/golden/reference)."""
     kat = json.load(open(golden_path("model_kat.json")))
+    excerpts = RG.model_excerpts()
     for name in kat:
-        path = os.path.join(REF_MODELS, f"{name}_model.json")
-        assert hashlib.sha256(open(path, "rb").read()).hexdigest() == kat[name]["sha256"]
-        m = w2x.Model.load_json(path)
-        for li, k in enumerate(kat[name]["layers"]):
-            w, b = m.params(li)
+        for li, text in excerpts[name].items():
+            li = int(li)
+            path = tmp_path / f"{name}_layer{li}.json"
+            path.write_text("[" + text + "]")
+            m = w2x.Model.load_json(str(path))
+            k = kat[name]["layers"][li]
+            w, b = m.params(0)
+            assert m.dims(0) == (*kat[name]["dims"][li], 3)
             assert float(w.reshape(-1)[0]) == k["w_first"] and float(w.reshape(-1)[-1]) == k["w_last"]
             assert float(b[0]) == k["b_first"] and float(b[-1]) == k["b_last"]
+            assert float(w.astype(np.float64).sum()) == k["w_sum64"]
             assert np.array_equal(w, oracle_models[name].weights[li])
             assert np.array_equal(b, oracle_models[name].biases[li])
 

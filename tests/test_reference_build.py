@@ -1,235 +1,144 @@
-"""The reference's OWN hot-path sources (src/modelHandler.cpp, src/convertRoutine.cpp), compiled where they lie
-against the OpenCV API shim in oracle/cvshim (oracle/Makefile -> oracle/_ref/libw2x_reference.so), pin the restated
-oracle and the golden vectors against the reference's real control flow: picojson model loading, the thread partition
-of Model::filter, the layer loop, replicate padding, the block-split arithmetic, crop and stitch.
+"""The reference's OWN hot-path sources (src/modelHandler.cpp, src/convertRoutine.cpp), compiled against the OpenCV API
+shim in oracle/cvshim, pin the restated oracle and the golden vectors against the reference's real control flow:
+picojson model loading, the thread partition of Model::filter, the layer loop, replicate padding, the block-split
+arithmetic, crop and stitch.
 
-The library is built only where /root/reference exists (the authoring container) and travels prebuilt to the GPU box;
-nothing here reads /root/reference at run time (the model JSONs are re-written from tests/golden/models)."""
-import os
-
+What that build computed on the seeded inputs below is stored in tests/golden/reference (recorded by
+oracle/reference_golden.py): digests of every output compared bit for bit, and the block order traced from its progress
+output.  The model JSONs it read were written from tests/golden/models."""
 import numpy as np
 import pytest
 
 from conftest import golden_path
-from oracle import reference_lib as R
-
-pytestmark = pytest.mark.skipif(not R.available(), reason="oracle/_ref/libw2x_reference.so not built (needs /root/reference at build time)")
+from oracle import reference_golden as RG
 
 # restated fp32 arithmetic of the shim vs OpenCV's SIMD kernels: re-association / FMA only
 SHIM_VS_CV2_TOL = 3e-6
 
 
 @pytest.fixture(scope="module")
-def ref_models(json_models):
-    R.configure(4, 9)                         # the reference's defaults: -j 4, 512x512 blocks
-    ms = {n: R.ReferenceModels(p) for n, p in json_models.items()}
-    yield ms
-    for m in ms.values():
-        m.close()
-    R.configure(4, 9)
+def ref():
+    return RG.load()
 
 
-def test_reference_loader_reads_the_model_files(ref_models, oracle_models):
-    for name, rm in ref_models.items():
-        assert rm.n == 7 and rm.dims == [tuple(d) for d in oracle_models[name].dims]
+def test_reference_loader_reads_the_model_files(ref, oracle_models):
+    for name, om in oracle_models.items():
+        assert len(ref["dims"][name]) == 7 and [tuple(d) for d in ref["dims"][name]] == [tuple(d) for d in om.dims]
 
 
 @pytest.mark.parametrize("name", ["scale2.0x", "noise1"])
 @pytest.mark.parametrize("n_job", [1, 3, 4])
-def test_oracle_is_bit_identical_to_the_reference_control_flow(ref_models, oracle_mod, oracle_models, name, n_job):
+def test_oracle_is_bit_identical_to_the_reference_control_flow(ref, oracle_mod, oracle_models, name, n_job):
     """convertWithModels, no-split path (src/convertRoutine.cpp:31-48), for every thread partition the reference forms
     (nOutputPlanes / nJob with the remainder on the last thread, src/modelHandler.cpp:46-65)."""
-    R.configure(n_job, 9)
-    for (w, h, seed) in ((1, 1, 11), (15, 13, 25), (37, 61, 47), (64, 48, 3)):
+    for (w, h, seed) in RG.CONVERT_SIZES:
         x = oracle_mod.seeded_plane(w, h, seed, "uniform")
-        y_ref = ref_models[name].convert(x, True)
         y_orc = oracle_models[name].convert(x, n_job=n_job)
-        assert y_ref.shape == (h, w)
-        assert np.array_equal(y_ref, y_orc), (w, h)
-    R.configure(4, 9)
+        assert y_orc.shape == (h, w)
+        assert RG.digest(y_orc) == ref["convert"][f"{name}/j{n_job}/{w}x{h}"], (w, h)
 
 
-def test_block_split_path_is_bit_identical(ref_models, oracle_mod, oracle_models):
+def test_block_split_path_is_bit_identical(ref, oracle_mod, oracle_models):
     """convertWithModelsBlockSplit (src/convertRoutine.cpp:84-169) with 64x64 blocks (threshold 64*64*3/2 = 6144 px):
     block rectangles, last-block handling, crop and stitch -- against the oracle's restatement and against no-split."""
-    R.configure(4, 6)
-    try:
-        om, rm = oracle_models["scale2.0x"], ref_models["scale2.0x"]
-        for (w, h, seed) in ((120, 90, 4), (101, 64, 5), (51, 121, 6), (150, 50, 7)):
-            assert w * h > 6144
-            x = oracle_mod.seeded_plane(w, h, seed, "uniform")
-            y_split = rm.convert(x, True)
-            assert np.array_equal(y_split, om.convert(x, True, block=(64, 64))), (w, h)
-            assert np.abs(y_split - rm.convert(x, False)).max() <= 1e-6, (w, h)
-        x = oracle_mod.seeded_plane(96, 64, 8, "uniform")            # exactly AT the threshold: the reference does not split
-        assert np.array_equal(rm.convert(x, True), om.convert(x, True, block=(64, 64)))
-    finally:
-        R.configure(4, 9)
+    om = oracle_models["scale2.0x"]
+    for (w, h, seed) in RG.SPLIT64_SIZES:
+        assert w * h > 6144
+        x = oracle_mod.seeded_plane(w, h, seed, "uniform")
+        y_split, y_nosplit = om.convert(x, True, block=(64, 64)), om.convert(x, False)
+        assert RG.digest(y_split) == ref["split64"][f"{w}x{h}"]["split"], (w, h)
+        assert RG.digest(y_nosplit) == ref["split64"][f"{w}x{h}"]["nosplit"], (w, h)
+        assert np.abs(y_split - y_nosplit).max() <= 1e-6, (w, h)
+    x = oracle_mod.seeded_plane(96, 64, 8, "uniform")            # exactly AT the threshold: the reference does not split
+    assert ref["split64"]["96x64"]["split"] == ref["split64"]["96x64"]["nosplit"]
+    assert RG.digest(om.convert(x, True, block=(64, 64))) == ref["split64"]["96x64"]["split"]
 
 
-def test_model_filter_per_layer(ref_models, oracle_models):
+def test_model_filter_per_layer(ref, oracle_models):
     """Model::filter of every layer on the golden 32x24 inputs: bit-equal to the oracle, within fp32 re-association of cv2."""
     z = np.load(golden_path("layers_32x24.npz"))
-    rm, om = ref_models["scale2.0x"], oracle_models["scale2.0x"]
-    for li in range(rm.n):
-        out = rm.filter(li, z[f"in{li}"])
-        assert np.array_equal(out, om.filter(li, z[f"in{li}"], n_job=4)), li
+    om = oracle_models["scale2.0x"]
+    assert len(ref["filter"]) == len(om)
+    for li in range(len(om)):
+        out = om.filter(li, z[f"in{li}"], n_job=4)
+        assert RG.digest(out) == ref["filter"][li], li
         assert np.abs(out - z[f"out{li}"]).max() <= SHIM_VS_CV2_TOL * max(1.0, float(np.abs(z[f"out{li}"]).max())), li
 
 
-def test_reference_control_flow_reproduces_the_cv2_golden_odd_sizes(ref_models, oracle_mod):
+def test_reference_control_flow_reproduces_the_cv2_golden_odd_sizes(ref, oracle_mod, oracle_models):
     z = np.load(golden_path("odd_sizes.npz"))
-    for (w, h) in ((1, 1), (15, 13), (37, 61)):
-        x = oracle_mod.seeded_plane(w, h, 10 + w, "uniform")
-        assert np.abs(ref_models["scale2.0x"].convert(x, True) - z[f"out_{w}x{h}"]).max() <= SHIM_VS_CV2_TOL
+    for (w, h) in RG.ODD_SIZES:
+        y = oracle_models["scale2.0x"].convert(oracle_mod.seeded_plane(w, h, 10 + w, "uniform"))
+        assert RG.digest(y) == ref["odd"][f"{w}x{h}"], (w, h)
+        assert np.abs(y - z[f"out_{w}x{h}"]).max() <= SHIM_VS_CV2_TOL
 
 
 @pytest.mark.slow
-def test_cfg1_256_reference_control_flow_vs_cv2_golden(ref_models, oracle_mod, ncpu):
+def test_cfg1_256_reference_control_flow_vs_cv2_golden(ref, oracle_mod, oracle_models, ncpu):
     """BASELINE config 1 through the reference's own code (shim arithmetic) against the output of real OpenCV arithmetic."""
-    R.configure(ncpu, 9)
-    try:
-        x = oracle_mod.seeded_plane(256, 256, 0, "uniform")
-        y = ref_models["scale2.0x"].convert(x, True)
-        g = np.load(golden_path("cfg1_scale2.0x_uniform.npy"))
-        assert np.abs(y - g).max() <= SHIM_VS_CV2_TOL
-    finally:
-        R.configure(4, 9)
+    y = oracle_models["scale2.0x"].convert(oracle_mod.seeded_plane(256, 256, 0, "uniform"), n_job=ncpu)
+    assert RG.digest(y) == ref["cfg1_scale2.0x_uniform"]
+    g = np.load(golden_path("cfg1_scale2.0x_uniform.npy"))
+    assert np.abs(y - g).max() <= SHIM_VS_CV2_TOL
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/models/scale2.0x_model.json"), reason="reference tree not present (GPU box)")
-def test_shipped_model_files_equal_the_golden_weights(ref_models, oracle_mod):
-    """Authoring container only: the reference's real JSON files through its real loader give the same output bits as the
-    JSON re-written from tests/golden/models (i.e. the committed weights ARE the shipped weights after double->float)."""
+def test_shipped_model_files_equal_the_golden_weights(ref, oracle_mod, oracle_models):
+    """The reference's real JSON files through its real loader give the same output bits as the committed weights
+    (i.e. the committed weights ARE the shipped weights after double->float)."""
     x = oracle_mod.seeded_plane(40, 30, 9, "smooth")
     for name in ("scale2.0x", "noise1", "noise2"):
-        real = R.ReferenceModels(f"/root/reference/models/{name}_model.json")
-        assert np.array_equal(real.convert(x, True), ref_models[name].convert(x, True)), name
-        real.close()
+        assert RG.digest(oracle_models[name].convert(x)) == ref["shipped_models_smooth_40x30"][name], name
 
 
-def _identity_model_json(path, n_layers=7):
-    """n_layers of 1 -> 1 planes, kernel = delta, bias 0: convertWithModels becomes the identity on positive input, cheap
-    enough to push the reference's block-split code through full-size planes."""
-    import json
-    layer = {"nInputPlane": 1, "nOutputPlane": 1, "kW": 3, "kH": 3, "weight": [[[[0, 0, 0], [0, 1, 0], [0, 0, 0]]]], "bias": [0.0]}
-    with open(path, "w") as f:
-        json.dump([layer] * n_layers, f)
-
-
-@pytest.mark.parametrize("w,h", [(512, 768), (513, 768), (768, 512), (499, 1), (1, 1), (1920, 1080), (3840, 2160), (4096, 4096), (1234, 3211)])
-def test_block_order_and_split_decision_of_the_reference_at_full_size(w2x, oracle_mod, tmp_path, w, h):
+@pytest.mark.parametrize("w,h", RG.FULL_SIZES)
+def test_block_order_and_split_decision_of_the_reference_at_full_size(w2x, ref, w, h):
     """BASELINE shapes through the reference's own convertWithModels with a 7-layer identity model: the split decision and
     the (c, r) processing order it prints (src/convertRoutine.cpp:25-26,100-134) are the product's w2x_requires_splitting /
     w2x_block_table, block for block; and the stitched output is the input (every pixel written exactly once)."""
-    import re
-    p = str(tmp_path / "identity.json")
-    _identity_model_json(p)
-    R.configure(4, 9)
-    rm = R.ReferenceModels(p)
-    x = oracle_mod.seeded_plane(w, h, 3, "uniform") + np.float32(0.25)
-    y, log = rm.convert_with_log(x, True)
-    rm.close()
-    assert np.array_equal(y, x)
-    blocks = [(int(c), int(r)) for c, r in re.findall(r"start process block \((\d+),(\d+)\)", log)]
+    run = ref["identity_full_size"][f"{w}x{h}"]
+    assert run["identity"]
+    blocks = [tuple(b) for b in run["blocks"]]
     assert (len(blocks) > 0) == w2x.requires_splitting(w, h)
     if blocks:
         tab, sc, sr = w2x.block_table(w, h, 7)
         assert [(int(t[1]), int(t[0])) for t in tab] == blocks          # table rows are (r, c, ...): reference order = r outer, c inner
         assert sc * sr == len(blocks)
-        assert log.count("Iteration #7...") == len(blocks)
+        assert run["iterations_7"] == len(blocks)
     else:
-        assert log.count("Iteration #7...") == 1
+        assert run["iterations_7"] == 1
 
 
-def test_block_arithmetic_against_the_reference_on_random_shapes(w2x, oracle_mod, tmp_path):
+def test_block_arithmetic_against_the_reference_on_random_shapes(w2x, ref):
     """Seeded random plane sizes x block sizes 2^5..2^9: the reference's own split decision and block order (traced through
     its progress output with the identity model) against w2x_requires_splitting / w2x_block_table -- including planes
     thinner than a block, last blocks of 1 row / column, and sizes exactly at the split threshold."""
-    import re
-    p = str(tmp_path / "identity.json")
-    _identity_model_json(p)
-    rm = R.ReferenceModels(p)
-    rng = np.random.default_rng(2024)
-    cases = []
-    for exp in (5, 6, 7, 9):
-        b = 1 << exp
-        for _ in range(8):
-            cases.append((exp, int(rng.integers(1, 6 * b)), int(rng.integers(1, 6 * b))))
-        thr = b * b * 3 // 2
-        cases += [(exp, thr // 8, 8), (exp, thr // 8 + 1, 8), (exp, b - 14, 3 * b), (exp, 2 * (b - 14) + 1, b)]   # at / just past the threshold, exact multiples of the stride
+    runs = ref["identity_random_shapes"]
     try:
-        for exp, w, h in cases:
-            if exp == 9 and w * h > 1500 * 1500:
-                w, h = min(w, 1500), min(h, 1500)
-            R.configure(4, exp)
+        for r in runs:
+            exp, w, h = r["exp"], r["w"], r["h"]
             w2x.set_block_size_exp2_square(exp)
-            x = oracle_mod.seeded_plane(w, h, exp, "uniform") + np.float32(0.25)
-            y, log = rm.convert_with_log(x, True)
-            assert np.array_equal(y, x), (exp, w, h)
-            blocks = [(int(c), int(r)) for c, r in re.findall(r"start process block \((\d+),(\d+)\)", log)]
+            assert r["identity"], (exp, w, h)
+            blocks = [tuple(b) for b in r["blocks"]]
             assert (len(blocks) > 0) == w2x.requires_splitting(w, h), (exp, w, h)
             if blocks:
                 tab, sc, sr = w2x.block_table(w, h, 7)
                 assert [(int(t[1]), int(t[0])) for t in tab] == blocks, (exp, w, h)
     finally:
-        R.configure(4, 9)
         w2x.set_block_size_exp2_square(9)
-        rm.close()
 
 
-def _fmt_number(rng, v):
-    """one of the spellings a JSON writer may produce for the double v"""
-    k = int(rng.integers(0, 8))
-    if k == 0:
-        return repr(float(v))
-    if k == 1:
-        return "%.17g" % v
-    if k == 2:
-        return "%.20e" % v
-    if k == 3:
-        return ("%.12E" % v).replace("E-0", "E-").replace("E+0", "E+")
-    if k == 4:
-        return "%.25f" % v
-    if k == 5:
-        return ("%.15g" % v).replace("e-0", "e-")
-    if k == 6:
-        return "%.9g" % v              # fewer digits than fp32 needs: a different double, same test (both loaders see it)
-    return "%.30g" % v
-
-
-def test_json_number_parsing_agrees_with_the_reference_loader(w2x, oracle_mod, tmp_path):
+def test_json_number_parsing_agrees_with_the_reference_loader(w2x, ref, oracle_mod, tmp_path):
     """The product's loader (csrc/model.cpp: hand-written JSON reader, std::from_chars, double -> float) against the
     reference's (picojson + strtod, src/modelHandler.cpp:74-115) on model files whose numbers are spelt every which way
     (long decimals, exponents, subnormal magnitudes, integers, -0), with shuffled keys and odd whitespace.  The weights
-    the product parsed are run through the oracle, the same file goes through the reference's own loader and
-    convertWithModels: one differing ulp in any weight or bias would show up in the output bits."""
-    rng = np.random.default_rng(77)
-    dims = [(1, 3), (3, 2), (2, 1)]
+    the product parsed are run through the oracle and compared with what the reference's own loader and
+    convertWithModels made of the same file: one differing ulp in any weight or bias would show up in the output bits."""
     x = oracle_mod.seeded_plane(23, 17, 5, "uniform")
-    R.configure(2, 9)
-    for trial in range(12):
-        layers = []
-        for (ci, co) in dims:
-            scale = 10.0 ** float(rng.integers(-3, 1))
-            w = rng.standard_normal((co, ci, 3, 3)) * scale
-            b = rng.standard_normal(co) * 0.1
-            if trial % 3 == 0:
-                w.flat[0], w.flat[1], w.flat[2], b[0] = 1.0, -0.0, 1e-42, 0.0          # integer-valued, negative zero, fp32-subnormal
-            wtxt = "[" + ",".join("[" + ",".join("[" + ",".join("[" + ", ".join(_fmt_number(rng, v) for v in row) + "]" for row in k) + "]" for k in o) + "]" for o in w) + "]"
-            btxt = "[" + ",\n ".join(_fmt_number(rng, v) for v in b) + "]"
-            items = [('"nInputPlane"', str(ci)), ('"nOutputPlane"', str(co)), ('"kW"', "3"), ('"kH"', "3.0" if trial % 2 else "3"), ('"weight"', wtxt), ('"bias"', btxt)]
-            order = rng.permutation(len(items))
-            sep = ["", " ", "\n", "\t  "][trial % 4]
-            layers.append("{" + ("," + sep).join(items[i][0] + sep + ":" + sep + items[i][1] for i in order) + "}")
-        path = str(tmp_path / f"fuzz{trial}.json")
-        with open(path, "w") as f:
-            f.write("[" + ",\n".join(layers) + "]\n")
-        m = w2x.Model.load_json(path)
-        ws, bs = zip(*[m.params(li) for li in range(len(dims))])
+    fuzz = ref["json_fuzz"]
+    for trial, text in enumerate(fuzz["texts"]):
+        path = tmp_path / f"fuzz{trial}.json"
+        path.write_text(text)
+        m = w2x.Model.load_json(str(path))
+        ws, bs = zip(*[m.params(li) for li in range(len(m))])
         ours = oracle_mod.OracleModel(list(ws), list(bs)).convert(x, n_job=2)
-        rm = R.ReferenceModels(path)
-        ref = rm.convert(x, True)
-        rm.close()
-        assert np.array_equal(ours, ref), trial
-    R.configure(4, 9)
+        assert RG.digest(ours) == fuzz["outputs"][trial], trial
