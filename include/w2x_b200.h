@@ -165,6 +165,38 @@ W2X_API int w2x_filter_layer(w2x_ctx *ctx, const w2x_model *model, int layer,
 W2X_API int w2x_filter_layer_device(w2x_ctx *ctx, const w2x_model *model, int layer,
                                     const float *d_in, float *d_out, int width, int height);
 
+/* ---- whole images on the device ----------------------------------------------------------- */
+/* What the reference's main.cpp does around its two convertWithModels calls with OpenCV, on the GPU: an 8-bit image is
+ * uploaded once, kept as three fp32 planes (Y, U, V) through every phase and downloaded once as 8-bit pixels.  Every result
+ * is bit-identical to the host plumbing (host/imgproc.hpp): same fp32/fp64 operations in the same order, no contraction.
+ * Pixels are interleaved 8-bit B,G,R (as imread loads them; channel 0 is treated as "R" like the reference does), rows
+ * `stride_bytes` apart (>= width*3).  An image belongs to one context: every operation queues on the context's stream
+ * (w2x_ctx_set_stream included); the calls that take HOST pointers are synchronous, the others are asynchronous.
+ * Destroy images before their context; w2x_ctx_destroy releases the device memory of images still alive, after which
+ * every call on them fails with W2X_ERR_ARG and w2x_image_destroy only frees the handle.  No CPU fallback: without a
+ * context every call fails with W2X_ERR_ARG. */
+typedef struct w2x_image w2x_image; /* Y, U, V fp32 planes on the context's device */
+/* imread + convertTo(CV_32F, 1/255) + cvtColor(RGB2YUV)   (src/main.cpp:74-76) */
+W2X_API int w2x_image_create(w2x_ctx *ctx, const uint8_t *bgr, int width, int height, size_t stride_bytes,
+                             w2x_image **out);
+/* Same from DEVICE pixels, asynchronous: d_bgr must stay valid until the context's stream has passed this call. */
+W2X_API int w2x_image_create_device(w2x_ctx *ctx, const uint8_t *d_bgr, int width, int height, size_t stride_bytes,
+                                    w2x_image **out);
+W2X_API void w2x_image_destroy(w2x_image *img);
+W2X_API int w2x_image_size(const w2x_image *img, int *width, int *height);
+/* Noise reduction phase (src/main.cpp:82-100): Y <- convertWithModels(Y), block_splitting = 1 */
+W2X_API int w2x_image_denoise(w2x_image *img, const w2x_model *model);
+/* One 2x scaling iteration (src/main.cpp:126-156): Y <- convertWithModels(nearest 2x of Y), U, V <- bicubic 2x */
+W2X_API int w2x_image_scale2x(w2x_image *img, const w2x_model *model);
+/* The shrink of non-power-of-two ratios (src/main.cpp:158-167): bilinear resize of all three planes */
+W2X_API int w2x_image_resize_linear(w2x_image *img, int width, int height);
+/* cvtColor(YUV2RGB) + convertTo(CV_8U, 255)   (src/main.cpp:171-172), to HOST pixels; synchronous */
+W2X_API int w2x_image_download(w2x_image *img, uint8_t *bgr, size_t stride_bytes);
+/* Same to DEVICE pixels, asynchronous */
+W2X_API int w2x_image_download_device(w2x_image *img, uint8_t *d_bgr, size_t stride_bytes);
+/* The fp32 planes to HOST memory (tests, callers that want float output); synchronous */
+W2X_API int w2x_image_planes(w2x_image *img, float *y, float *u, float *v, size_t stride_bytes);
+
 /* ---- multi-GPU row-band mode (one process per GPU; the caller moves the halo rows) ----------- */
 /* A plane of `height` rows is cut into contiguous bands, one per rank.  Each rank calls
  * w2x_band_begin with ITS band of the input plus up to n_layers rows of real neighbour data

@@ -17,7 +17,7 @@ The directory name is not a valid Python identifier; load it with
 (tests/conftest.py, bench.py and __graft_entry__.py do exactly this through w2x_loader.py).
 """
 from .capi import (  # noqa: F401
-    ENGINE_AUTO, ENGINE_FP32, ENGINE_TC, PRECISION_F16X3, PRECISION_F16_F8X2, WALK_BLOCKS, WALK_FUSED, Band, Context, DevBytes, Model, Multi, Slab, W2xError,
+    ENGINE_AUTO, ENGINE_FP32, ENGINE_TC, PRECISION_F16X3, PRECISION_F16_F8X2, WALK_BLOCKS, WALK_FUSED, Band, Context, DevBytes, Image, Model, Multi, Slab, W2xError,
     block_table, get_block_size, get_jobs, lib, lib_path, requires_splitting, set_block_size,
     set_block_size_exp2_square, set_jobs, version,
 )

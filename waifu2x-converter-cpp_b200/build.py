@@ -26,7 +26,8 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-I", os.path.join(ROOT, "include"), "-I", CSRC,
           "-Xcompiler", "-fPIC,-fvisibility=hidden,-Wall,-Wextra"] + os.environ.get("W2X_BUILD_DEFS", "").split()
-LIB_SOURCES = ["model.cpp", "geometry.cpp", "kernels_fp32.cu", "kernels_tc.cu", "engine.cu", "engine_band.cu"]
+LIB_SOURCES = ["model.cpp", "geometry.cpp", "kernels_fp32.cu", "kernels_tc.cu", "image.cu", "engine.cu", "engine_band.cu",
+               "engine_image.cu"]
 
 
 def _newer(target, deps):

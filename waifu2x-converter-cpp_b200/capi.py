@@ -39,6 +39,8 @@ ABI_SYMBOLS = (
     "w2x_multi_set_precision", "w2x_multi_set_log", "w2x_multi_convert_plane", "w2x_multi_convert_tiles",
     "w2x_host_alloc", "w2x_host_free", "w2x_ctx_forget_model", "w2x_slab_create", "w2x_slab_destroy", "w2x_slab_export",
     "w2x_slab_connect", "w2x_slab_connect_local", "w2x_slab_convert", "w2x_slab_convert_async", "w2x_slab_synchronize",
+    "w2x_image_create", "w2x_image_create_device", "w2x_image_destroy", "w2x_image_size", "w2x_image_denoise",
+    "w2x_image_scale2x", "w2x_image_resize_linear", "w2x_image_download", "w2x_image_download_device", "w2x_image_planes",
 )
 BAND_BLOB_BYTES = 320
 
@@ -147,6 +149,17 @@ def lib():
     L.w2x_multi_set_log.argtypes = [vp, LOG_FN, vp]
     L.w2x_multi_convert_plane.argtypes = [vp, vp, vp, ci, ci, cs, vp, cs, ci]
     L.w2x_multi_convert_tiles.argtypes = [vp, vp, C.POINTER(vp), C.POINTER(vp), ci, ci, ci, cs, cs]
+    L.w2x_image_create.argtypes = [vp, vp, ci, ci, cs, C.POINTER(vp)]
+    L.w2x_image_create_device.argtypes = [vp, vp, ci, ci, cs, C.POINTER(vp)]
+    L.w2x_image_destroy.argtypes = [vp]
+    L.w2x_image_destroy.restype = None
+    L.w2x_image_size.argtypes = [vp, C.POINTER(ci), C.POINTER(ci)]
+    L.w2x_image_denoise.argtypes = [vp, vp]
+    L.w2x_image_scale2x.argtypes = [vp, vp]
+    L.w2x_image_resize_linear.argtypes = [vp, ci, ci]
+    L.w2x_image_download.argtypes = [vp, vp, cs]
+    L.w2x_image_download_device.argtypes = [vp, vp, cs]
+    L.w2x_image_planes.argtypes = [vp, vp, vp, vp, cs]
     L.w2x_debug_set_host_bands.argtypes = [vp, ci]
     L.w2x_debug_set_pair.argtypes = [vp, ci]
     L.w2x_debug_set_fuse_last.argtypes = [vp, ci]
@@ -389,6 +402,71 @@ class Context:
 
     def filter_layer_device(self, model: Model, layer, d_in, d_out, w, h):
         _check(lib().w2x_filter_layer_device(self._h, model._h, layer, C.c_void_p(d_in), C.c_void_p(d_out), w, h))
+
+
+# ---- whole images on the device -----------------------------------------------------------------
+class Image:
+    """w2x_image_*: an 8-bit B,G,R image kept on the context's device as fp32 Y, U, V planes through the reference
+    main.cpp's phases (denoise, 2x scaling, bilinear shrink), bit-identical to the host plumbing.
+
+    Image(ctx, bgr)                          from a host uint8 array [h][w][3] (rows may be strided)
+    Image.from_device(ctx, ptr, w, h, stride)  from device pixels (e.g. a CUDA uint8 tensor's data_ptr()), asynchronous"""
+
+    def __init__(self, ctx: Context, bgr=None, _handle=None):
+        self._ctx = ctx                      # the context must outlive the image
+        if _handle is not None:
+            self._h = _handle
+            return
+        x = np.asarray(bgr, np.uint8)
+        if x.ndim != 3 or x.shape[2] != 3:
+            raise ValueError("bgr must be [h][w][3] uint8")
+        if x.strides[2] != 1 or x.strides[1] != 3:
+            x = np.ascontiguousarray(x)
+        h = C.c_void_p()
+        _check(lib().w2x_image_create(ctx._h, C.c_void_p(x.ctypes.data), x.shape[1], x.shape[0], x.strides[0], C.byref(h)))
+        self._h = h
+
+    @classmethod
+    def from_device(cls, ctx: Context, d_bgr, width, height, stride_bytes):
+        h = C.c_void_p()
+        _check(lib().w2x_image_create_device(ctx._h, C.c_void_p(d_bgr), width, height, stride_bytes, C.byref(h)))
+        return cls(ctx, _handle=h)
+
+    def close(self):
+        if getattr(self, "_h", None) and _lib is not None:
+            _lib.w2x_image_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    def size(self):
+        """-> (width, height)"""
+        w, h = C.c_int(), C.c_int()
+        _check(lib().w2x_image_size(self._h, C.byref(w), C.byref(h)))
+        return w.value, h.value
+
+    def denoise(self, model: Model): _check(lib().w2x_image_denoise(self._h, model._h))
+    def scale2x(self, model: Model): _check(lib().w2x_image_scale2x(self._h, model._h))
+    def resize_linear(self, width, height): _check(lib().w2x_image_resize_linear(self._h, width, height))
+
+    def download(self, out=None):
+        """-> uint8 [h][w][3] B,G,R (host, synchronous)"""
+        w, h = self.size()
+        if out is None:
+            out = np.empty((h, w, 3), np.uint8)
+        _check(lib().w2x_image_download(self._h, C.c_void_p(out.ctypes.data), out.strides[0]))
+        return out
+
+    def download_device(self, d_bgr, stride_bytes):
+        _check(lib().w2x_image_download_device(self._h, C.c_void_p(d_bgr), stride_bytes))
+
+    def planes(self):
+        """-> float32 [3][h][w]: Y, U, V (host, synchronous)"""
+        w, h = self.size()
+        out = np.empty((3, h, w), np.float32)
+        _check(lib().w2x_image_planes(self._h, C.c_void_p(out[0].ctypes.data), C.c_void_p(out[1].ctypes.data),
+                                      C.c_void_p(out[2].ctypes.data), w * 4))
+        return out
 
 
 # ---- row-band session with a halo exchange between layers ---------------------------------------

@@ -138,13 +138,6 @@ void emit_reference_progress(w2x_ctx *ctx, int w, int h, int n_layers, bool spli
     }
 }
 
-struct LogMute {   // silences the per-launch lines while a caller that already emitted the reference's sequence runs the layers
-    w2x_ctx *ctx;
-    bool prev;
-    explicit LogMute(w2x_ctx *c, bool on) : ctx(c), prev(c->log_muted) { if (on) c->log_muted = true; }
-    ~LogMute() { ctx->log_muted = prev; }
-};
-
 int pick_engine(w2x_ctx *ctx, const w2x_model *m) {
     int e = ctx->engine;
     if (e == W2X_ENGINE_AUTO) e = m->tc_eligible ? W2X_ENGINE_TC : W2X_ENGINE_FP32;
@@ -446,6 +439,7 @@ void w2x_ctx_destroy(w2x_ctx *ctx) {
     if (!ctx) return;
     DeviceGuard g(ctx->device);
     cudaStreamSynchronize(ctx->stream);
+    release_images(ctx);
     for (auto &kv : ctx->models) free_dev_model(kv.second);
     for (int i = 0; i < 2; i++) {
         cudaFree(ctx->buf[i]);

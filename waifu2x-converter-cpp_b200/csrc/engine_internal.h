@@ -71,6 +71,7 @@ struct w2x_ctx {
     cudaEvent_t ev_in[8] = {}, ev_done[8] = {};
     int host_bands = 0;                                   // 0 = automatic (up to 4 bands of >= 512 rows), 1 = no pipelining
     unsigned long long *prof_buf = nullptr;   // [16 layers][PROF_MAX_CTAS][PROF_WORDS], debug profile
+    std::vector<w2x_image *> images;          // live w2x_image handles of this context (engine_image.cu)
 };
 
 // One rank's rows of a plane (w2x_band_*): every intermediate activation keeps only the band's rows plus one halo row per
@@ -144,6 +145,16 @@ int convert_device(w2x_ctx *ctx, const w2x_model *m, const float *d_in, int w, i
 
 int tiles_enqueue_compute(w2x_ctx *ctx, const w2x_model *model, const float *const *in_tiles, int n_tiles, int width, int height, size_t in_stride_bytes);
 int tiles_enqueue_download(w2x_ctx *ctx, float *const *out_tiles, int n_tiles, int width, int height, size_t out_stride_bytes);
+
+struct LogMute {   // silences the per-launch lines while a caller that already emitted the reference's sequence runs the layers
+    w2x_ctx *ctx;
+    bool prev;
+    explicit LogMute(w2x_ctx *c, bool on) : ctx(c), prev(c->log_muted) { if (on) c->log_muted = true; }
+    ~LogMute() { ctx->log_muted = prev; }
+};
+
+// engine_image.cu: w2x_ctx_destroy releases the device buffers of the context's images that are still alive
+void release_images(w2x_ctx *ctx);
 
 struct NvtxRange {    // a named range on the calling thread's timeline (nsys / ncu --nvtx), e.g. "w2x L3", "w2x halo exchange"
     explicit NvtxRange(const char *name) { nvtxRangePushA(name); }

@@ -35,6 +35,16 @@ cudaError_t launch_copy2d(const float *in, long in_stride_floats, float *out, lo
 cudaError_t launch_conv3x3_fp32(const float *in, float *out, const float *wgt, const float *bias, int Cin, int Cout,
                                 int W, int H, cudaStream_t s);
 
+// ---- image.cu: whole-image plumbing on dense planar fp32 Y, U, V planes (bit-identical to host/imgproc.hpp) -----------
+// interleaved 8-bit B,G,R (row stride in bytes) <-> three dense w x h planes
+cudaError_t launch_bgr8_to_yuv(const uint8_t *bgr, size_t stride_bytes, int w, int h, float *Y, float *U, float *V, cudaStream_t s);
+cudaError_t launch_yuv_to_bgr8(const float *Y, const float *U, const float *V, int w, int h, uint8_t *bgr, size_t stride_bytes,
+                               cudaStream_t s);
+cudaError_t launch_resize_nearest(const float *src, int sw, int sh, float *dst, int dw, int dh, cudaStream_t s);
+struct ResizePlanes { const float *src[3]; float *dst[3]; };
+// bicubic (A = -0.75) or bilinear resize of n_planes (<= 3) dense planes of one geometry
+cudaError_t launch_resize(const ResizePlanes &p, int n_planes, int sw, int sh, int dw, int dh, bool cubic, cudaStream_t s);
+
 // ---- kernels_tc.cu ----------------------------------------------------------------------------
 namespace tc {
 constexpr int REGION = 16;          // a tile-set covers REGION x REGION output pixels (two 8x16 M-tiles)

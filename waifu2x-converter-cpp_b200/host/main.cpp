@@ -1,7 +1,8 @@
 // main.cpp -- drop-in command line of waifu2x-converter-cpp (reference src/main.cpp) on top of the GPU hot path.
 // Same flags, defaults, progress messages, output naming and exit codes; the two convertWithModels calls
 // (src/main.cpp:96,148) go to libw2x_b200.so through host/w2xc.hpp, everything around them is restated from
-// src/main.cpp line by line with host/imgproc.hpp + host/imageio.hpp standing in for OpenCV.
+// src/main.cpp line by line with host/imgproc.hpp + host/imageio.hpp standing in for OpenCV.  With one GPU the colour and
+// resize steps run on the device instead (w2xc::DeviceImage), bit-identical to imgproc.hpp.
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -177,8 +178,35 @@ int main(int argc, char **argv) {
         leave(-1);
     }
     const double t_read = now();
-    w2ximg::Image3f image = w2ximg::from_u8(in8.bgr.data(), in8.width, in8.height);
-    w2ximg::rgb2yuv(image);
+    // The image runs on one of two paths, picked at the first convertWithModels call site (after that phase's model file has
+    // loaded, so that every message and exit code stays where the reference has it):
+    //   device: one GPU -- w2xc::DeviceImage keeps Y, U, V on the GPU from the upload to the download (bit-identical);
+    //   host:   --gpus > 1 (w2x_multi_convert_plane takes host planes), no device, or no conversion at all --
+    //           host/imgproc.hpp around convertWithModels, as below.
+    // W2X_CLI_HOST_PLUMBING=1 forces the host path (A/B measurements, the bit-identity tests).
+    w2ximg::Image3f image;
+    bool image_ready = false;
+    auto host_image = [&]() -> w2ximg::Image3f & {                                        // :75-76, deferred to first use
+        if (!image_ready) {
+            image = w2ximg::from_u8(in8.bgr.data(), in8.width, in8.height);
+            w2ximg::rgb2yuv(image);
+            image_ready = true;
+        }
+        return image;
+    };
+    w2xc::DeviceImage dev;
+    bool on_device = false, path_chosen = false;
+    // sets on_device on the first call; *failed = the upload of the device path failed (reported like a failed conversion)
+    auto choose_path = [&](bool *failed) {
+        *failed = false;
+        if (path_chosen) return;
+        path_chosen = true;
+        if (std::getenv("W2X_CLI_HOST_PLUMBING") || w2xc::gpuRuntime::numberOfGpus() > 1) return;
+        wait_for_gpu();
+        if (!w2xc::gpuRuntime::context() || w2xc::gpuRuntime::multi()) return;                // no device: the host path fails as today
+        on_device = true;
+        *failed = !dev.create(in8.bgr.data(), in8.width, in8.height);
+    };
 
     w2xc::modelUtility::getInstance().setNumberOfJobs(std::atoi(cmd.get("jobs").c_str()));   // :79
     // (-j bounds the reference's filter threads; here it bounds the host image plumbing's row workers, the GPU does the filtering)
@@ -188,15 +216,24 @@ int main(int argc, char **argv) {
         std::string modelFileName = modelDir + "/noise" + std::to_string(nrLevel) + "_model.json";
         std::vector<std::unique_ptr<w2xc::Model>> models;
         if (!w2xc::modelUtility::generateModelFromJSON(modelFileName, models)) leave(-1);
-        w2xc::Plane imageY = plane_of(image, 0), out;
-        wait_for_gpu();
-        const double t0 = now();
-        // The reference ignores the return value here (:96) because a failing layer has already ended the process inside
-        // convertWithModelsBasic (src/convertRoutine.cpp:69: std::exit(-1)).  The library never exits, so the same outcome
-        // is produced here: no device, out of memory or a CUDA error must not write the un-denoised image with exit code 0.
-        if (!w2xc::convertWithModels(imageY, out, models) || out.empty()) leave(-1);
-        t_conv += now() - t0;
-        w2ximg::set_channel(image, 0, out.data, out.stride_bytes / 4);
+        bool failed;
+        choose_path(&failed);
+        if (failed) leave(-1);
+        if (on_device) {
+            const double t0 = now();
+            if (!dev.denoise(models)) leave(-1);
+            t_conv += now() - t0;
+        } else {
+            w2xc::Plane imageY = plane_of(host_image(), 0), out;
+            wait_for_gpu();
+            const double t0 = now();
+            // The reference ignores the return value here (:96) because a failing layer has already ended the process inside
+            // convertWithModelsBasic (src/convertRoutine.cpp:69: std::exit(-1)).  The library never exits, so the same outcome
+            // is produced here: no device, out of memory or a CUDA error must not write the un-denoised image with exit code 0.
+            if (!w2xc::convertWithModels(imageY, out, models) || out.empty()) leave(-1);
+            t_conv += now() - t0;
+            w2ximg::set_channel(image, 0, out.data, out.stride_bytes / 4);
+        }
     }
 
     // ===== scaling phase ===== (:104-169)
@@ -211,9 +248,21 @@ int main(int argc, char **argv) {
         std::cout << "start scaling" << std::endl;
         for (int nIteration = 0; nIteration < iterTimesTwiceScaling; nIteration++) {
             std::cout << "#" << std::to_string(nIteration + 1) << " 2x scaling..." << std::endl;
-            const int w2 = image.width * 2, h2 = image.height * 2;
-            w2xc::Plane imageY = plane_of_nearest(image, 0, w2, h2), out;                 // :135-139 (only the Y plane of the nearest image is used)
-            w2ximg::Image3f bicubic = w2ximg::resize(image, w2, h2, w2ximg::CUBIC);      // :144
+            bool failed;
+            choose_path(&failed);
+            if (on_device) {
+                const double t0 = now();
+                if (failed || !dev.scale2x(models)) {                                       // nearest + bicubic + conv + merge, :135-155
+                    std::cerr << "w2xc::convertWithModels : something error has occured.\nstop." << std::endl;
+                    leave(1);
+                }
+                t_conv += now() - t0;
+                continue;
+            }
+            w2ximg::Image3f &im = host_image();
+            const int w2 = im.width * 2, h2 = im.height * 2;
+            w2xc::Plane imageY = plane_of_nearest(im, 0, w2, h2), out;                    // :135-139 (only the Y plane of the nearest image is used)
+            w2ximg::Image3f bicubic = w2ximg::resize(im, w2, h2, w2ximg::CUBIC);         // :144
             wait_for_gpu();
             const double t0 = now();
             if (!w2xc::convertWithModels(imageY, out, models)) {
@@ -225,14 +274,30 @@ int main(int argc, char **argv) {
             image = std::move(bicubic);
         }
         if (shrinkRatio != 0.0) {                                                           // :158-167
-            int lw = static_cast<int>(static_cast<double>(image.width * shrinkRatio));
-            int lh = static_cast<int>(static_cast<double>(image.height * shrinkRatio));
-            image = w2ximg::resize(image, lw, lh, w2ximg::LINEAR);
+            const int cw = on_device ? dev.width() : host_image().width, ch = on_device ? dev.height() : image.height;
+            int lw = static_cast<int>(static_cast<double>(cw * shrinkRatio));
+            int lh = static_cast<int>(static_cast<double>(ch * shrinkRatio));
+            if (on_device) {
+                if (!dev.resizeLinear(lw, lh)) leave(-1);
+            } else {
+                image = w2ximg::resize(image, lw, lh, w2ximg::LINEAR);
+            }
         }
     }
 
-    w2ximg::yuv2rgb(image);                                                                 // :171
-    std::vector<uint8_t> out8 = w2ximg::to_u8(image);                                       // :172
+    std::vector<uint8_t> out8;
+    int out_w, out_h;
+    if (on_device) {                                                                        // :171-172 on the GPU, one download
+        out_w = dev.width();
+        out_h = dev.height();
+        out8.resize((size_t)out_w * out_h * 3);
+        if (!dev.download(out8.data())) leave(-1);
+    } else {
+        w2ximg::yuv2rgb(host_image());                                                      // :171
+        out8 = w2ximg::to_u8(image);                                                        // :172
+        out_w = image.width;
+        out_h = image.height;
+    }
     std::string outputFileName = cmd.get("output_file");
     if (outputFileName == "(auto)") {                                                       // :173-189
         outputFileName = inputFile;
@@ -244,7 +309,7 @@ int main(int argc, char **argv) {
         outputFileName += ".png";
     }
     const double t_write0 = now();
-    if (!w2xio::imwrite(outputFileName, out8.data(), image.width, image.height)) {
+    if (!w2xio::imwrite(outputFileName, out8.data(), out_w, out_h)) {
         std::cerr << "Error : couldn't write " << outputFileName << std::endl;
         leave(-1);
     }

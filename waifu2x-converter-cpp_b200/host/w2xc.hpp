@@ -91,6 +91,11 @@ public:
     }
     static void warmup() { (void)instance(); }                // create the runtime (CUDA context) now, silently
     static w2x_multi *multi() { return instance().multi_; }   // nullptr with one GPU
+    // the number of GPUs the runtime is (or will be) created with, without creating it
+    static int numberOfGpus() {
+        const char *ng = std::getenv("W2X_GPUS");
+        return requested() > 0 ? requested() : (ng ? std::atoi(ng) : 1);
+    }
 private:
     static int &requested() { static int n = 0; return n; }
     static bool &created() { static bool c = false; return c; }
@@ -100,9 +105,9 @@ private:
     std::string error_;
     gpuRuntime() {
         created() = true;
-        const char *dev = std::getenv("W2X_DEVICE"), *ng = std::getenv("W2X_GPUS");
+        const char *dev = std::getenv("W2X_DEVICE");
         const int first = dev ? std::atoi(dev) : 0;
-        int n = requested() > 0 ? requested() : (ng ? std::atoi(ng) : 1);
+        const int n = numberOfGpus();
         if (n > 1) {
             std::vector<int> ids;
             for (int i = 0; i < n; i++) ids.push_back(first + i);
@@ -131,8 +136,19 @@ class Model {
     std::shared_ptr<w2x_model> file_;
     int layer_ = 0;
     friend class modelUtility;
+    friend class DeviceImage;
     friend bool convertWithModels(Plane &, Plane &, std::vector<std::unique_ptr<Model>> &, bool);
     Model(std::shared_ptr<w2x_model> f, int layer) : file_(std::move(f)), layer_(layer) {}
+    // the model file of `models`, which must be its layers in order (as generateModelFromJSON produces them); nullptr + message if not
+    static w2x_model *fileOf(std::vector<std::unique_ptr<Model>> &models) {
+        for (size_t i = 0; i < models.size(); i++)
+            if (models[i]->file_ != models[0]->file_ || models[i]->layer_ != (int)i ||
+                (int)models.size() != w2x_model_layer_count(models[0]->file_.get())) {
+                std::cerr << "Error : convertWithModels : models must be the layers of one model file, in order." << std::endl;
+                return nullptr;
+            }
+        return models.empty() ? nullptr : models[0]->file_.get();
+    }
 
 public:
     int getNInputPlanes() { int a = 0; w2x_model_layer_dims(file_.get(), layer_, &a, nullptr, nullptr); return a; }
@@ -260,13 +276,7 @@ public:
 inline bool convertWithModels(Plane &inputPlane, Plane &outputPlane, std::vector<std::unique_ptr<Model>> &models,
                               bool blockSplitting = true) {
     w2x_ctx *ctx = gpuRuntime::context();
-    if (!ctx || models.empty() || inputPlane.empty()) return false;
-    for (size_t i = 0; i < models.size(); i++)
-        if (models[i]->file_ != models[0]->file_ || models[i]->layer_ != (int)i ||
-            (int)models.size() != w2x_model_layer_count(models[0]->file_.get())) {
-            std::cerr << "Error : convertWithModels : models must be the layers of one model file, in order." << std::endl;
-            return false;
-        }
+    if (!ctx || models.empty() || inputPlane.empty() || !Model::fileOf(models)) return false;
     if (outputPlane.data == inputPlane.data || outputPlane.width != inputPlane.width || outputPlane.height != inputPlane.height)
         outputPlane.create(inputPlane.width, inputPlane.height);
     static struct Printer {
@@ -287,6 +297,50 @@ inline bool convertWithModels(Plane &inputPlane, Plane &outputPlane, std::vector
     }
     return true;
 }
+
+// Not in the reference: a whole image on the GPU (w2x_image_*), for the single-GPU runtime.  What the reference's main.cpp
+// does with cv::Mat around its convertWithModels calls (src/main.cpp:74-76, 82-100, 126-167, 171-172) happens on the device,
+// bit-identical to the host plumbing: upload 8-bit B,G,R once, denoise / scale2x / resizeLinear, download once.  Every
+// method returns once the work has finished; on failure it prints w2x_last_error() and returns false.
+class DeviceImage {
+    w2x_image *img_ = nullptr;
+    static bool report() {
+        std::cerr << w2x_last_error() << std::endl;
+        return false;
+    }
+    bool finish(int rc) { return rc == W2X_OK && w2x_ctx_synchronize(gpuRuntime::context()) == W2X_OK ? true : report(); }
+    bool convert(std::vector<std::unique_ptr<Model>> &models, int (*fn)(w2x_image *, const w2x_model *)) {
+        w2x_ctx *ctx = gpuRuntime::context();
+        w2x_model *m = Model::fileOf(models);
+        if (!ctx || !img_ || !m) return false;
+        static struct Printer {
+            static void line(const char *l, void *) { std::cout << l << std::endl; }
+        } printer;
+        (void)printer;
+        w2x_ctx_set_log(ctx, &Printer::line, nullptr);   // "Iteration #k..." / "start process block (c,r) ...", as convertWithModels
+        return finish(fn(img_, m));
+    }
+
+public:
+    DeviceImage() {}
+    DeviceImage(const DeviceImage &) = delete;
+    DeviceImage &operator=(const DeviceImage &) = delete;
+    ~DeviceImage() { w2x_image_destroy(img_); }
+    // 8-bit B,G,R pixels, rows stride_bytes apart (0 = width * 3), on the runtime's single-GPU context
+    bool create(const uint8_t *bgr, int width, int height, size_t stride_bytes = 0) {
+        w2x_ctx *ctx = gpuRuntime::context();
+        if (!ctx) return false;
+        w2x_image_destroy(img_);
+        img_ = nullptr;
+        return w2x_image_create(ctx, bgr, width, height, stride_bytes ? stride_bytes : (size_t)width * 3, &img_) == W2X_OK ? true : report();
+    }
+    bool denoise(std::vector<std::unique_ptr<Model>> &models) { return convert(models, w2x_image_denoise); }
+    bool scale2x(std::vector<std::unique_ptr<Model>> &models) { return convert(models, w2x_image_scale2x); }
+    bool resizeLinear(int width, int height) { return img_ && finish(w2x_image_resize_linear(img_, width, height)); }
+    bool download(uint8_t *bgr) { return img_ && (w2x_image_download(img_, bgr, (size_t)width() * 3) == W2X_OK ? true : report()); }
+    int width() const { int w = 0; w2x_image_size(img_, &w, nullptr); return w; }
+    int height() const { int h = 0; w2x_image_size(img_, nullptr, &h); return h; }
+};
 
 #ifdef W2X_WITH_OPENCV
 // The reference's own signatures (src/modelHandler.hpp:87-88, src/convertRoutine.hpp:25-28) on cv::Mat: CV_32FC1 planes are
